@@ -2,6 +2,7 @@
 """bench.py — the render-prep hot path on N B200s (one process per GPU).
 
     python bench.py --gpus 1 --steps K --warmup W                 # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                         # + the last timed frame's outputs as DIR/<name>.npy
     torchrun --nproc-per-node N ... bench.py --gpus N ...          # weak scaling, NCCL all-gather of visible lists
     python bench.py --impl reference --gpus N --steps K --warmup W # the reference's CPU algorithm (oracle port), host cores
 
@@ -53,6 +54,10 @@ B_BONE = 196
 B_VERT = 68
 UPLOAD_FIELD = {"rot": "changed_rot", "trs": "changed_trs", "m16": "changed_m16"}
 UPLOAD_BYTES = {"rot": 16, "trs": 40, "m16": 64}
+# --dump-outputs: how many nodes / skinned meshes of the last timed frame are written (about 30 MB at C4, under the 64 MB cap)
+DUMP_NODES = 1 << 18
+DUMP_UNITS = 8
+DUMP_MAX_BYTES = 64 << 20
 
 
 def peaks():
@@ -405,6 +410,43 @@ def oracle_frusta(n_frusta: int):
     return [ob.frustum_from_vp(ob.mat4_mul(ob.perspective(1.0, float(np.pi / 2), 0.01, 120.0), ob.look_at_rh((0, 0, 0), look, up))) for look, up in faces[:n_frusta]]
 
 
+def dump_outputs(ctx, sc, n_frusta, out_dir, log):
+    """Write what the last timed frame computed, as a caller of fyx_render_prep receives it, to out_dir/<name>.npy (float32 or
+    float64): for a fixed, seeded sample of nodes their global matrices, world boxes and per-frustum visibility; the length
+    and id sum of every visible list; the palettes and skinned streams of a few skinned meshes.  The visible lists are
+    compared as sets (their order is not part of the result), and two builds run with the same arguments get the same
+    inputs, so their dumps compare array for array."""
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+    from sampled_parity import SortedList
+
+    ctx.sync()
+    rng = np.random.default_rng(SEED)
+    nodes = np.unique(rng.integers(0, sc.capacity, DUMP_NODES)).astype(np.uint32)
+    gid = sc.global_index[nodes]
+    lists = [SortedList(ctx.get_visible(f, copy=False)) for f in range(n_frusta)]
+    out = {
+        "node_index": gid.astype(np.float64),
+        "global_matrices": ctx.get_global_matrices(nodes),
+        "world_aabbs": ctx.get_world_aabbs(nodes),
+        "visible": np.stack([sl.contains(gid) for sl in lists], axis=1).astype(np.float32),
+        "visible_counts": np.array([sl.a.size for sl in lists], np.float64),
+        "visible_id_sums": np.array([sl.a.sum(dtype=np.uint64) for sl in lists], np.float64),
+    }
+    if sc.n_units:  # surface id = unit index (load_scene adds them in order)
+        units = np.unique(np.concatenate([[0, sc.n_units - 1], rng.integers(0, sc.n_units, DUMP_UNITS - 2)]))
+        skinned = [ctx.get_skinned(int(u)) for u in units]
+        out["skinned_unit_index"] = units.astype(np.float64)
+        out["palettes"] = np.stack([ctx.get_palette(int(u)) for u in units])
+        out["skinned_positions"] = np.stack([p for p, _ in skinned])
+        out["skinned_normals"] = np.stack([n for _, n in skinned])
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"dumped {len(out)} arrays ({total / 1e6:.1f} MB) of the last timed frame to {out_dir}")
+
+
 def parity_block(ctx, sc, fb, frusta, upload, world, rank, dist, log):
     """Sampled-oracle check of the context that was just timed (outside every timed region; the oracle is the checker,
     never on the product path).  One more synchronous frame with animation frame 0, then per rank: >= 5 000 sampled
@@ -455,10 +497,11 @@ def parity_block(ctx, sc, fb, frusta, upload, world, rank, dist, log):
     return out
 
 
-def measure(args, wname, strong, steps, env, full):
+def measure(args, wname, strong, steps, env, full, dump_dir=None):
     """All timed regions (+ the parity block) of one workload on this rank's GPU.  `strong`: the workload's sizes are
     the WHOLE job, sharded over the ranks (strong scaling); otherwise they are per GPU (weak scaling).
-    `full`: also the secondary modes (static+skeletons, device animation) and the synchronous e2e."""
+    `full`: also the secondary modes (static+skeletons, device animation) and the synchronous e2e.
+    `dump_dir`: write the outputs of the last all-dirty timed frame there (dump_outputs) before anything else runs."""
     import torch
 
     import fyrox_b200 as fb
@@ -574,6 +617,8 @@ def measure(args, wname, strong, steps, env, full):
     launches0 = ctx.kernel_launch_count()
     total_ms = timed(step_device, steps)
     launches = ctx.kernel_launch_count() - launches0
+    if dump_dir:
+        dump_outputs(ctx, sc, len(frusta), dump_dir, log)
     e2e_sync_ms = timed(step_e2e, steps, pass_index=True) if full else None
     for _ in range(2):
         run_e2e_pipelined(3)
@@ -713,7 +758,7 @@ def run_cuda(args):
 
     w = WORKLOADS[args.workload]
     strong_main = args.workload == "C5"
-    r = measure(args, args.workload, strong_main, args.steps, env, full=True)
+    r = measure(args, args.workload, strong_main, args.steps, env, full=True, dump_dir=args.dump_outputs if rank == 0 else None)
     # BASELINE.json configs[4] / north_star: the 100 M-node config, STRONG scaling (the whole job is fixed, sharded N ways)
     c5 = None
     if args.workload == "C4" and not args.no_c5:
@@ -804,8 +849,14 @@ def main():
     ap.add_argument("--no-full-frame", action="store_true", help="reference arm: skip the one frame of the full workload that follows the bounded sample")
     ap.add_argument("--no-parity", action="store_true", help="skip the sampled-oracle check that follows the timed regions")
     ap.add_argument("--no-c5", action="store_true", help="skip the strong-scaling C5 measurement that follows the default C4 workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                    "(a fixed, seeded sample; rank 0's context when N > 1)")
     ap.add_argument("--verbose", action="store_true")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm's timed path")
     # OpenMP workers (scene generator, multi-core CPU baseline) that wait at a barrier should sleep, not spin: the host is
     # shared with the other ranks and possibly quota-limited (must be set before libgomp is loaded)
     os.environ.setdefault("OMP_WAIT_POLICY", "PASSIVE")

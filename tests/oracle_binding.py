@@ -79,7 +79,11 @@ def lib() -> C.CDLL:
     if _lib is not None:
         return _lib
     src = os.path.join(ORACLE_DIR, "fyrox_oracle.c")
-    if not os.path.exists(ORACLE_LIB) or (os.path.exists(src) and os.path.getmtime(src) > os.path.getmtime(ORACLE_LIB)):
+    # a stale library is rebuilt only where the tree is writable: a read-only install (bench.py's CPU baseline and parity
+    # block) uses what build() made, whatever mtimes a copy of the tree left on the sources
+    missing = not os.path.exists(ORACLE_LIB)
+    stale = not missing and os.path.exists(src) and os.path.getmtime(src) > os.path.getmtime(ORACLE_LIB)
+    if missing or (stale and os.access(ORACLE_DIR, os.W_OK)):
         build()
     L = C.CDLL(ORACLE_LIB)
     vp = C.c_void_p

@@ -33,6 +33,12 @@ def test_c1_runs_whole_on_the_cpu():
     assert d["config"]["sample"].startswith("100000 nodes, 0 skinned meshes") and d["value"] > 0
 
 
+def test_arguments_that_cannot_be_honoured_are_refused():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--workload", "tiny", *extra], capture_output=True, text=True, timeout=120)
+        assert out.returncode == 2 and out.stdout.strip() == "", extra
+
+
 def test_other_ranks_of_the_reference_arm_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--impl", "reference", "--gpus", "2", "--workload", "tiny"],

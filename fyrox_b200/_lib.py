@@ -236,6 +236,9 @@ SYMBOLS = {
     "fyx_get_bone_matrix_blocks_device": (C.c_int32, [ctx_p, C.c_uint32, C.c_void_p]),
     "fyx_set_blend_shapes": (C.c_int32, [ctx_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p]),
     "fyx_set_blend_shape_weights": (C.c_int32, [ctx_p, C.c_uint32, C.c_uint32, C.c_void_p]),
+    "fyx_set_skinned_tangents": (C.c_int32, [ctx_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32]),
+    "fyx_get_skinned_tangents": (C.c_int32, [ctx_p, C.c_uint32, C.c_void_p]),
+    "fyx_get_skinned_tangents_device": (C.c_int32, [ctx_p, C.c_uint32, C.POINTER(C.c_void_p)]),
     "fyx_allgather_visible": (C.c_int32, [ctx_p]),
     "fyx_comm_mode": (C.c_uint32, [ctx_p]),
     "fyx_comm_get_stats": (C.c_int32, [ctx_p, C.c_void_p]),

@@ -246,6 +246,37 @@ class Context:
         assert w is None or w.size == r.shape[0]
         self._chk(self._lib.fyx_set_blend_shapes(self._h, surface_id, r.shape[0], r.ctypes.data_as(C.c_void_p), r.shape[1], _ptr(w)))
 
+    def set_skinned_tangents(self, surface_id: int, verts, tangent_offset: int = 32, stride: int = None):
+        """Skin the tangents of a surface too (standard.shader:197-200): verts = its VertexBuffer bytes again (tangent = f32 x4 at
+        tangent_offset; 32 in AnimatedVertex), stride = bytes per vertex (default: the layout the surface was added with for a
+        numpy array of records, else 68); verts may also be a raw (pinned) address.  verts = None turns them off.  Must come before
+        set_blend_shapes."""
+        if verts is None:
+            self._chk(self._lib.fyx_set_skinned_tangents(self._h, surface_id, None, 0, 0))
+            return
+        if isinstance(verts, np.ndarray):
+            verts = np.ascontiguousarray(verts)
+            nv = self._surfaces[surface_id][1]
+            if stride is None:
+                stride = verts.nbytes // nv if nv else ANIMATED_VERTEX_LAYOUT.stride
+            assert verts.nbytes >= nv * stride
+            vptr = verts.ctypes.data_as(C.c_void_p)
+        else:  # raw address of n_verts records
+            vptr = C.c_void_p(int(verts))
+            stride = ANIMATED_VERTEX_LAYOUT.stride if stride is None else stride
+        self._chk(self._lib.fyx_set_skinned_tangents(self._h, surface_id, vptr, stride, tangent_offset))
+
+    def get_skinned_tangents(self, surface_id: int) -> np.ndarray:
+        nv = self._surfaces[surface_id][1]
+        out = np.empty((nv, 3), dtype=np.float32)
+        self._chk(self._lib.fyx_get_skinned_tangents(self._h, surface_id, out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def get_skinned_tangents_device(self, surface_id: int):
+        p = C.c_void_p()
+        self._chk(self._lib.fyx_get_skinned_tangents_device(self._h, surface_id, C.byref(p)))
+        return p.value
+
     def set_blend_shape_weights(self, surface_id: int, weights):
         w = np.ascontiguousarray(weights, dtype=np.float32)
         self._chk(self._lib.fyx_set_blend_shape_weights(self._h, surface_id, w.size, _ptr(w)))

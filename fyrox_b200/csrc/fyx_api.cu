@@ -40,6 +40,11 @@ struct Surface {
     uint32_t n_shapes = 0, bs_blocks = 0, bs_cap = 0; // shapes, 128-vertex blocks per shape, capacity of the region in shape blocks
     uint64_t bs_off = 0;                               // first shape block of the region
     uint32_t w_off = 0, w_cap = 0;
+    // skinned tangents (fyx_set_skinned_tangents): on, and the surface's regions (kept when turned off, reused when turned on again)
+    bool tangents = false;
+    uint32_t tan_blk = FYX_NONE;  // first block in b_tblk
+    uint32_t tan_quad0 = 0;       // first 4-vertex group in b_otan
+    uint32_t bst_off = 0, bst_cap = 0; // tangent blend-shape region in b_bst: first shape block, capacity in shape blocks
 };
 
 enum { EV_START = 0, EV_UPLOAD, EV_UPDATE, EV_CULL, EV_PALETTE, EV_SKIN, EV_READBACK, EV_COUNT };
@@ -176,6 +181,9 @@ struct fyx_ctx {
     uint64_t bs_used = 0;         // shape blocks handed out
     uint32_t bs_w_used = 0;
     bool any_blend_shapes = false;
+    DevBuf b_tblk, b_otan, b_bst; // skinned tangents: input blocks, output stream, blend-shape offsets (only tangent surfaces have any)
+    uint64_t tan_blocks_used = 0, tan_quads_used = 0, bst_used = 0;
+    bool any_tangents = false;
     DevBuf b_fold_node, b_fold_begin, b_fold_bone, b_fold_stale_idx, b_late_slot, b_stale_pos;
     std::vector<uint32_t> dfs_rank; // optional: pre-order rank of every node in the reference's DFS (fyx_set_dfs_order)
     uint32_t n_late = 0;
@@ -702,7 +710,7 @@ extern "C" void fyx_destroy(fyx_ctx *c)
     inst_free(c);
     anim_free(c);
     DevBuf *bufs[] = {&c->b_vis, &c->b_parent, &c->b_flags, &c->b_mask, &c->b_gidx, &c->b_slot_of_node, &c->d_stage, &c->b_statics, &c->b_trs, &c->b_vblk,
-                      &c->b_ms_range, &c->b_ms_bundle, &c->b_ms_skin, &c->b_prune, &c->b_sf_rng, &c->b_opos, &c->b_onrm, &c->b_bs, &c->b_bs_w, &c->b_surf_of_slot, &c->b_surf_bones, &c->b_palette, &c->b_bone_slot, &c->b_tiles, &c->b_fold_node,
+                      &c->b_ms_range, &c->b_ms_bundle, &c->b_ms_skin, &c->b_prune, &c->b_sf_rng, &c->b_opos, &c->b_onrm, &c->b_bs, &c->b_bs_w, &c->b_tblk, &c->b_otan, &c->b_bst, &c->b_surf_of_slot, &c->b_surf_bones, &c->b_palette, &c->b_bone_slot, &c->b_tiles, &c->b_fold_node,
                       &c->b_fold_begin, &c->b_fold_bone, &c->b_fold_stale_idx, &c->b_late_slot, &c->b_stale_pos, &c->b_counts_packed, &c->b_counts_all};
     for (DevBuf *b : bufs) dev_free(*b);
     for (int i = 0; i < 3; ++i) {
@@ -1354,6 +1362,9 @@ void rebuild_skin_arrays(fyx_ctx *c)
     sk.onrm = c->b_onrm.as<float>();
     sk.bs = c->b_bs.as<uint2>();
     sk.bs_w = c->b_bs_w.as<float>();
+    sk.tblk = c->b_tblk.as<float4>();
+    sk.otan = c->b_otan.as<float>();
+    sk.bst = c->b_bst.as<uint2>();
 }
 
 constexpr uint32_t kTileQuads = 2048; // up to 8192 vertices per tile (a 5k-vertex surface is one tile)
@@ -1393,6 +1404,9 @@ int32_t commit_surfaces(fyx_ctx *c)
                 tl.bs_blocks = sf.bs_blocks;
                 tl.w_off = sf.w_off;
                 tl.local_quad0 = t * per;
+                tl.tan_blk = sf.tangents ? sf.tan_blk : FYX_NONE;
+                tl.tan_quad0 = sf.tan_quad0;
+                tl.bst_off = sf.bst_off;
                 tiles.push_back(tl);
             }
         }
@@ -1459,6 +1473,8 @@ int32_t commit_surfaces(fyx_ctx *c)
     c->n_tiles = (uint32_t)tiles.size();
     c->any_blend_shapes = false;
     for (const Surface &sf : c->surfaces) c->any_blend_shapes |= sf.n_shapes != 0 && sf.n_verts != 0;
+    c->any_tangents = false;
+    for (const Surface &sf : c->surfaces) c->any_tangents |= sf.tangents && sf.n_verts != 0;
     c->max_bones = 0;
     for (const Surface &sf : c->surfaces)
         if (sf.n_verts) c->max_bones = std::max(c->max_bones, sf.n_bones);
@@ -1583,6 +1599,13 @@ extern "C" int32_t fyx_set_blend_shapes(fyx_ctx *c, uint32_t sid, uint32_t n_sha
         sf.w_cap = n_shapes;
         c->bs_w_used += n_shapes;
     }
+    if (sf.tangents && need > sf.bst_cap) { // the same for the tangent offsets of a tangent surface
+        if (c->bst_used + need > 0xFFFFFFFFull) return fail(c, FYX_ERR_OUT_OF_MEMORY, "blend-shape storage exhausted");
+        if ((rc = dev_ensure(c, c->b_bst, (c->bst_used + need) * kBstBlockU2 * sizeof(uint2), true))) return rc;
+        sf.bst_off = (uint32_t)c->bst_used;
+        sf.bst_cap = (uint32_t)need;
+        c->bst_used += need;
+    }
     sf.n_shapes = n_shapes;
     sf.bs_blocks = bs_blocks;
     rebuild_skin_arrays(c);
@@ -1592,9 +1615,57 @@ extern "C" int32_t fyx_set_blend_shapes(fyx_ctx *c, uint32_t sid, uint32_t n_sha
     if ((rc = stage_to_device(c, records, (size_t)n_shapes * layer_stride * 18, w.data(), (size_t)n_shapes * 4, false, &d_rec, &d_w))) return rc;
     launch_bs_layout(c->stream, sf.n_verts, n_shapes, layer_stride, static_cast<const uint16_t *>(d_rec), c->b_bs.as<uint2>() + sf.bs_off * kBsBlockU2, bs_blocks);
     c->launches++;
+    if (sf.tangents) {
+        launch_bs_tan_layout(c->stream, sf.n_verts, n_shapes, layer_stride, static_cast<const uint16_t *>(d_rec),
+                             c->b_bst.as<uint2>() + (size_t)sf.bst_off * kBstBlockU2, bs_blocks);
+        c->launches++;
+    }
     CU(cudaMemcpyAsync(c->b_bs_w.as<float>() + sf.w_off, d_w, (size_t)n_shapes * 4, cudaMemcpyDeviceToDevice, c->stream));
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(c->stream)); // `w` and the staging buffer are free again
+    return FYX_OK;
+}
+
+// Skinned tangents of a surface (standard.shader:197-200): its VertexBuffer bytes again, tangent = f32 x4 at tangent_offset
+extern "C" int32_t fyx_set_skinned_tangents(fyx_ctx *c, uint32_t sid, const void *verts, uint32_t stride, uint32_t tangent_offset)
+{
+    if (!c) return FYX_ERR_INVALID_ARGUMENT;
+    if (sid >= c->surfaces.size()) return fail(c, FYX_ERR_INVALID_ARGUMENT, "surface id %u out of range", sid);
+    Surface &sf = c->surfaces[sid];
+    if (!verts) {
+        if (sf.tangents) c->tables_dirty = true;
+        sf.tangents = false;
+        return FYX_OK;
+    }
+    if (stride % 4 || tangent_offset % 4) return fail(c, FYX_ERR_INVALID_ARGUMENT, "vertex stride and tangent offset must be multiples of 4");
+    if ((uint64_t)tangent_offset + 16 > stride) return fail(c, FYX_ERR_INVALID_ARGUMENT, "tangent (16 B at %u) outside the %u-byte vertex", tangent_offset, stride);
+    if (sf.n_shapes)
+        return fail(c, FYX_ERR_STATE, "surface %u already has blend shapes: call fyx_set_skinned_tangents before fyx_set_blend_shapes", sid);
+    CU(cudaSetDevice(c->device));
+    int32_t rc;
+    const uint64_t quads = ((uint64_t)sf.n_verts + 3) / 4, blocks = (quads + 31) / 32;
+    if (sf.tan_blk == FYX_NONE && sf.n_verts) { // the surface's regions, kept for the rest of its life
+        if (c->tan_blocks_used + blocks > 0xFFFFFFFFull || c->tan_quads_used + quads > 0xFFFFFFFFull)
+            return fail(c, FYX_ERR_OUT_OF_MEMORY, "tangent storage exhausted");
+        if ((rc = dev_ensure(c, c->b_tblk, (c->tan_blocks_used + blocks) * kTblkStride * sizeof(float4), true))) return rc;
+        if ((rc = dev_ensure(c, c->b_otan, (c->tan_quads_used + quads) * 48, true))) return rc;
+        sf.tan_blk = (uint32_t)c->tan_blocks_used;
+        sf.tan_quad0 = (uint32_t)c->tan_quads_used;
+        c->tan_blocks_used += blocks;
+        c->tan_quads_used += quads;
+        rebuild_skin_arrays(c);
+    }
+    if (sf.n_verts) {
+        void *d_v = nullptr;
+        if ((rc = stage_to_device(c, verts, (size_t)sf.n_verts * stride, nullptr, 0, false, &d_v, nullptr))) return rc;
+        launch_tan_deinterleave(c->stream, sf.n_verts, static_cast<const unsigned char *>(d_v), stride, tangent_offset,
+                                c->b_tblk.as<float4>() + (size_t)sf.tan_blk * kTblkStride);
+        c->launches++;
+        CU(cudaGetLastError());
+        CU(cudaStreamSynchronize(c->stream)); // the staging buffer is free again
+    }
+    sf.tangents = true;
+    c->tables_dirty = true;
     return FYX_OK;
 }
 
@@ -1749,7 +1820,7 @@ extern "C" int32_t fyx_skin(fyx_ctx *c)
     if (rc) return rc;
     CU(cudaEventRecord(c->ev[EV_START], c->stream));
     if (c->n_tiles) {
-        launch_skin(c->stream, c->sk, c->b_tiles.as<SkinTile>(), c->n_tiles, c->max_bones, c->any_blend_shapes);
+        launch_skin(c->stream, c->sk, c->b_tiles.as<SkinTile>(), c->n_tiles, c->max_bones, c->any_blend_shapes, c->any_tangents);
         c->launches++;
     }
     CU(cudaEventRecord(c->ev[EV_SKIN], c->stream));
@@ -1901,7 +1972,7 @@ extern "C" int32_t fyx_render_prep(fyx_ctx *c, const fyx_frame_desc *fr)
     }
     if (stage_events) CU(cudaEventRecord(c->ev[EV_PALETTE], s));
     if (fr->do_skin && c->n_tiles) {
-        launch_skin(s, c->sk, c->b_tiles.as<SkinTile>(), c->n_tiles, c->max_bones, c->any_blend_shapes);
+        launch_skin(s, c->sk, c->b_tiles.as<SkinTile>(), c->n_tiles, c->max_bones, c->any_blend_shapes, c->any_tangents);
         c->launches++;
     }
     if (stage_events) CU(cudaEventRecord(c->ev[EV_SKIN], s));
@@ -2077,6 +2148,30 @@ extern "C" int32_t fyx_get_skinned_device(fyx_ctx *c, uint32_t sid, const float 
     const Surface &sf = c->surfaces[sid];
     if (d_pos) *d_pos = c->b_opos.as<float>() + 3 * sf.vert_off;
     if (d_nrm) *d_nrm = c->b_onrm.as<float>() + 3 * sf.vert_off;
+    return FYX_OK;
+}
+
+extern "C" int32_t fyx_get_skinned_tangents(fyx_ctx *c, uint32_t sid, float *out_tan3)
+{
+    if (!c) return FYX_ERR_INVALID_ARGUMENT;
+    if (sid >= c->surfaces.size()) return fail(c, FYX_ERR_INVALID_ARGUMENT, "surface id %u out of range", sid);
+    const Surface &sf = c->surfaces[sid];
+    if (!sf.tangents) return fail(c, FYX_ERR_STATE, "surface %u has no skinned tangents (fyx_set_skinned_tangents)", sid);
+    if (!sf.n_verts) return FYX_OK;
+    if (!out_tan3) return fail(c, FYX_ERR_INVALID_ARGUMENT, "out_tan3 is NULL");
+    CU(cudaSetDevice(c->device));
+    CU(cudaMemcpyAsync(out_tan3, c->b_otan.as<float>() + 12 * (size_t)sf.tan_quad0, (size_t)sf.n_verts * 12, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return FYX_OK;
+}
+
+extern "C" int32_t fyx_get_skinned_tangents_device(fyx_ctx *c, uint32_t sid, const float **d_tan3)
+{
+    if (!c) return FYX_ERR_INVALID_ARGUMENT;
+    if (sid >= c->surfaces.size()) return fail(c, FYX_ERR_INVALID_ARGUMENT, "surface id %u out of range", sid);
+    const Surface &sf = c->surfaces[sid];
+    if (!sf.tangents) return fail(c, FYX_ERR_STATE, "surface %u has no skinned tangents (fyx_set_skinned_tangents)", sid);
+    if (d_tan3) *d_tan3 = sf.n_verts ? c->b_otan.as<float>() + 12 * (size_t)sf.tan_quad0 : nullptr;
     return FYX_OK;
 }
 

@@ -65,6 +65,13 @@ struct SkinArrays {
     // (px,py,pz,nx,ny,nz) x 32 groups x 4 halfs = 1536 B per (shape, block); weights = BlendShape::weight / 100
     const uint2 *bs;
     const float *bs_w;
+    // skinned tangents (optional, per surface; fyx_set_skinned_tangents): tangent xyz in blocks of 128 vertices x 3 rows
+    // (tx,ty,tz) of 32 float4 (1536 B), the same row / group convention as vblk but counted from the surface's first
+    // vertex; the output otan is one packed-xyz stream per tangent surface (padded to a multiple of 4 vertices).  Their
+    // blend-shape offsets (halfs 6-8 of each record) in blocks of 3 rows x 32 groups x 4 halfs = 768 B per (shape, block).
+    const float4 *tblk;
+    float *otan;
+    const uint2 *bst;
 };
 
 struct SkinTile {
@@ -78,10 +85,21 @@ struct SkinTile {
     uint32_t bs_blocks;   // 128-vertex blocks per shape
     uint32_t w_off;       // first weight in bs_w
     uint32_t local_quad0; // the tile's first group relative to the surface's first group
-    uint32_t pad[3];
+    // tangents of the surface (tan_blk = FYX_NONE: none)
+    uint32_t tan_blk;     // first block of the surface in tblk
+    uint32_t tan_quad0;   // first group of the surface in otan (12 floats per group)
+    uint32_t bst_off;     // index of (shape 0, block 0) of the surface's tangent offsets, in units of kBstBlockU2
 };
-constexpr uint32_t kBsBlockU2 = 6 * 32; // uint2 per (shape, block)
+static_assert(sizeof(SkinTile) == 48, "SkinTile stays 48 B");
+constexpr uint32_t kBsBlockU2 = 6 * 32;  // uint2 per (shape, block)
+constexpr uint32_t kBstBlockU2 = 3 * 32; // uint2 per (shape, block) of the tangent offsets
+constexpr int kTblkStride = 3 * 32;      // float4 per tangent block of 128 vertices
+// records (9 halfs per vertex and layer) -> blocked rows: halfs 0-5 into bs (6 rows), halfs 6-8 into bst (3 rows)
 void launch_bs_layout(cudaStream_t s, uint32_t n_verts, uint32_t n_shapes, uint32_t layer_stride, const uint16_t *d_records, uint2 *d_dst, uint32_t bs_blocks);
+void launch_bs_tan_layout(cudaStream_t s, uint32_t n_verts, uint32_t n_shapes, uint32_t layer_stride, const uint16_t *d_records, uint2 *d_dst,
+                          uint32_t bs_blocks);
+// VertexBuffer bytes -> the surface's tangent blocks (tblk points at its first block)
+void launch_tan_deinterleave(cudaStream_t s, uint32_t n_verts, const unsigned char *d_bytes, uint32_t stride, uint32_t tangent_offset, float4 *tblk);
 
 struct FoldArrays {
     uint32_t n; // skinned mesh nodes
@@ -192,7 +210,8 @@ void launch_cull_lights(cudaStream_t s, const NodeArrays &a, const CullParams &c
 void launch_fold_bones(cudaStream_t s, const NodeArrays &a, const FoldArrays &fa, const CullParams *cull);
 void launch_snapshot_bones(cudaStream_t s, const NodeArrays &a, uint32_t n_late, const uint32_t *late_slot, float4 *stale_pos);
 void launch_palette(cudaStream_t s, const NodeArrays &a, const SkinArrays &sk);
-void launch_skin(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles, uint32_t max_bones, bool blend_shapes);
+void launch_skin(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles, uint32_t max_bones, bool blend_shapes,
+                 bool tangents);
 
 void launch_scatter_locals(cudaStream_t s, const NodeArrays &a, uint32_t count, const uint32_t *d_idx,
                            const float *d_m16, const uint32_t *slot_of_node, uint32_t n_nodes, uint32_t *d_err);

@@ -1005,27 +1005,34 @@ __device__ __forceinline__ void skin_fill_palette(float4 *s_pal, const float *pa
     }
 }
 
-// four vertices (one thread's group) from registers to the two output streams
-template <int S, int LOG2C>
+// four vertices (one thread's group) from registers to the two output streams; TAN: also their tangents to the third
+// (standard.shader:197-200 skins inputTangent.xyz as the normal, acc += (mat3(P[idx_k]) * t) * w_k, k in order).  The
+// tangent reuses the palette rows the position and normal just read: (tx, ty) go through the packed pipe as the normal's
+// (x, y), tz is the scalar third row, r_z = (m_20*tx + m_21*ty) + m_22*tz (one rounding per product and sum).
+template <int S, int LOG2C, bool TAN = false>
 __device__ __forceinline__ void skin_quad(const float4 *s_pal, const uint32_t lane, const float4 x4, const float4 y4, const float4 z4,
                                           const float4 nx4, const float4 ny4, const float4 nz4, const float4 w0, const float4 w1,
                                           const float4 w2, const float4 w3, const uint4 iq, float4 *po, float4 *no,
-                                          const PackedConsts kc)
+                                          const PackedConsts kc, const float4 tx4 = float4{}, const float4 ty4 = float4{},
+                                          const float4 tz4 = float4{}, float4 *to = nullptr)
 {
     constexpr int C = 1 << LOG2C;
     constexpr int PL = S * C;
     const float px[4] = {x4.x, x4.y, x4.z, x4.w}, py[4] = {y4.x, y4.y, y4.z, y4.w}, pz[4] = {z4.x, z4.y, z4.z, z4.w};
     const float nx[4] = {nx4.x, nx4.y, nx4.z, nx4.w}, ny[4] = {ny4.x, ny4.y, ny4.z, ny4.w}, nz[4] = {nz4.x, nz4.y, nz4.z, nz4.w};
+    const float tx[4] = {tx4.x, tx4.y, tx4.z, tx4.w}, ty[4] = {ty4.x, ty4.y, ty4.z, ty4.w}, tz[4] = {tz4.x, tz4.y, tz4.z, tz4.w};
     // w_k holds weight k of the four vertices
     const float wk4[4][4] = {{w0.x, w1.x, w2.x, w3.x}, {w0.y, w1.y, w2.y, w3.y}, {w0.z, w1.z, w2.z, w3.z}, {w0.w, w1.w, w2.w, w3.w}};
     const uint32_t iv[4] = {iq.x, iq.y, iq.z, iq.w};
-    float ox[4], oy[4], oz[4], mx[4], my[4], mz[4];
+    float ox[4], oy[4], oz[4], mx[4], my[4], mz[4], ux[4], uy[4], uz[4];
 #pragma unroll
     for (int v = 0; v < 4; ++v) {
         const float2 pxx = make_float2(px[v], px[v]), pyy = make_float2(py[v], py[v]), pzz = make_float2(pz[v], pz[v]);
         const float2 nxx = make_float2(nx[v], nx[v]), nyy = make_float2(ny[v], ny[v]), nzz = make_float2(nz[v], nz[v]);
         const float2 pnx = make_float2(px[v], nx[v]), pny = make_float2(py[v], ny[v]), pnz = make_float2(pz[v], nz[v]);
         float2 acc_p = make_float2(0.0f, 0.0f), acc_n = make_float2(0.0f, 0.0f), acc_z = make_float2(0.0f, 0.0f);
+        float2 acc_t = make_float2(0.0f, 0.0f);
+        float acc_tz = 0.0f;
         const float *wk = wk4[v];
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -1043,9 +1050,18 @@ __device__ __forceinline__ void skin_quad(const float4 *s_pal, const uint32_t la
             float2 z = add2(add2(mul2(pnx, make_float2(Z.x, Z.x), kc), mul2(pny, make_float2(Z.y, Z.y), kc), kc), mul2(pnz, make_float2(Z.z, Z.z), kc), kc);
             z.x = FYX_ADD(z.x, Z.w);
             acc_z = add2(acc_z, mul2(z, ww, kc), kc);
+            if (TAN) {
+                // tangent (sx, sy) = (m_i0*tx + m_i1*ty) + m_i2*tz;  sz = (m_20*tx + m_21*ty) + m_22*tz
+                const float2 txx = make_float2(tx[v], tx[v]), tyy = make_float2(ty[v], ty[v]), tzz = make_float2(tz[v], tz[v]);
+                const float2 sxy = add2(add2(mul2(lo2(A), txx, kc), mul2(hi2(A), tyy, kc), kc), mul2(lo2(B), tzz, kc), kc);
+                acc_t = add2(acc_t, mul2(sxy, ww, kc), kc);
+                const float sz = FYX_ADD(FYX_ADD(FYX_MUL(Z.x, tx[v]), FYX_MUL(Z.y, ty[v])), FYX_MUL(Z.z, tz[v]));
+                acc_tz = FYX_ADD(acc_tz, FYX_MUL(sz, wk[k]));
+            }
         }
         ox[v] = acc_p.x; oy[v] = acc_p.y; oz[v] = acc_z.x;
         mx[v] = acc_n.x; my[v] = acc_n.y; mz[v] = acc_z.y;
+        ux[v] = acc_t.x; uy[v] = acc_t.y; uz[v] = acc_tz;
     }
     st_stream(po + 0, make_float4(ox[0], oy[0], oz[0], ox[1]));
     st_stream(po + 1, make_float4(oy[1], oz[1], ox[2], oy[2]));
@@ -1053,6 +1069,11 @@ __device__ __forceinline__ void skin_quad(const float4 *s_pal, const uint32_t la
     st_stream(no + 0, make_float4(mx[0], my[0], mz[0], mx[1]));
     st_stream(no + 1, make_float4(my[1], mz[1], mx[2], my[2]));
     st_stream(no + 2, make_float4(mz[2], mx[3], my[3], mz[3]));
+    if (TAN) {
+        st_stream(to + 0, make_float4(ux[0], uy[0], uz[0], ux[1]));
+        st_stream(to + 1, make_float4(uy[1], uz[1], ux[2], uy[2]));
+        st_stream(to + 2, make_float4(uz[2], ux[3], uy[3], uz[3]));
+    }
 }
 
 // two vertices (half of a four-vertex group) per thread: 22 input registers instead of 44 — k_skin2 trades wider loads for
@@ -1163,7 +1184,25 @@ __device__ __forceinline__ void apply_blend_shapes(const SkinArrays &sk, const S
     }
 }
 
-// BlendShapesContainer's records (9 halfs per vertex and layer: position, normal, tangent) -> the blocked device layout
+// the tangent offsets of a tangent surface (fyx_set_skinned_tangents): halfs 6-8 of each record, added in shape order
+// exactly as the normal offsets above (standard.shader:167-173 adds offsets.tangent * weight to inputTangent.xyz)
+__device__ __forceinline__ void apply_blend_shapes_tan(const SkinArrays &sk, const SkinTile &T, const uint32_t e, float4 &tx4, float4 &ty4, float4 &tz4)
+{
+    const uint2 *r0 = sk.bst + ((size_t)T.bst_off + (e >> 5)) * kBstBlockU2 + (e & 31u);
+    const size_t shape_stride = (size_t)T.bs_blocks * kBstBlockU2;
+    for (uint32_t sidx = 0; sidx < T.n_shapes; ++sidx) {
+        const float w = sk.bs_w[T.w_off + sidx];
+        const uint2 *r = r0 + sidx * shape_stride;
+        const uint2 htx = r[0 * 32], hty = r[1 * 32], htz = r[2 * 32];
+        bs_axpy(tx4, htx, w);
+        bs_axpy(ty4, hty, w);
+        bs_axpy(tz4, htz, w);
+    }
+}
+
+// BlendShapesContainer's records (9 halfs per vertex and layer: position, normal, tangent) -> the blocked device layout:
+// halfs [H0, H0 + NH) of every record into NH rows per (shape, block) (H0 = 0, NH = 6: bs; H0 = 6, NH = 3: bst)
+template <int H0, int NH>
 __global__ void __launch_bounds__(kBlock) k_bs_layout(const uint32_t n_verts, const uint32_t n_shapes, const uint32_t layer_stride,
                                                       const uint16_t *rec, uint16_t *dst, const uint32_t bs_blocks)
 {
@@ -1171,26 +1210,42 @@ __global__ void __launch_bounds__(kBlock) k_bs_layout(const uint32_t n_verts, co
     const uint64_t per_shape = (uint64_t)bs_blocks * 128;
     if (t >= per_shape * n_shapes) return;
     const uint32_t sidx = (uint32_t)(t / per_shape), v = (uint32_t)(t % per_shape);
-    uint16_t h[6] = {0, 0, 0, 0, 0, 0};
+    uint16_t h[NH] = {};
     if (v < n_verts) {
-        const uint16_t *r = rec + ((size_t)sidx * layer_stride + v) * 9;
-        for (int k = 0; k < 6; ++k) h[k] = r[k];
+        const uint16_t *r = rec + ((size_t)sidx * layer_stride + v) * 9 + H0;
+        for (int k = 0; k < NH; ++k) h[k] = r[k];
     }
-    // (shape, block) = 6 rows x 32 groups x 4 halfs
-    uint16_t *blk = dst + ((size_t)sidx * bs_blocks + (v >> 7)) * (kBsBlockU2 * 4);
+    // (shape, block) = NH rows x 32 groups x 4 halfs
+    uint16_t *blk = dst + ((size_t)sidx * bs_blocks + (v >> 7)) * (NH * 32 * 4);
     const uint32_t g = (v >> 2) & 31u, j = v & 3u;
-    for (int k = 0; k < 6; ++k) blk[(k * 32 + g) * 4 + j] = h[k];
+    for (int k = 0; k < NH; ++k) blk[(k * 32 + g) * 4 + j] = h[k];
+}
+
+template <int H0, int NH>
+static void launch_bs_layout_t(cudaStream_t s, uint32_t n_verts, uint32_t n_shapes, uint32_t layer_stride, const uint16_t *d_records, uint2 *d_dst,
+                               uint32_t bs_blocks)
+{
+    if (!n_shapes || !bs_blocks) return;
+    k_bs_layout<H0, NH><<<(unsigned)(((uint64_t)bs_blocks * 128 * n_shapes + kBlock - 1) / kBlock), kBlock, 0, s>>>(
+        n_verts, n_shapes, layer_stride, d_records, reinterpret_cast<uint16_t *>(d_dst), bs_blocks);
 }
 
 void launch_bs_layout(cudaStream_t s, uint32_t n_verts, uint32_t n_shapes, uint32_t layer_stride, const uint16_t *d_records, uint2 *d_dst, uint32_t bs_blocks)
 {
-    if (!n_shapes || !bs_blocks) return;
-    k_bs_layout<<<(unsigned)(((uint64_t)bs_blocks * 128 * n_shapes + kBlock - 1) / kBlock), kBlock, 0, s>>>(n_verts, n_shapes, layer_stride, d_records,
-                                                                                                        reinterpret_cast<uint16_t *>(d_dst), bs_blocks);
+    static_assert(kBsBlockU2 * 4 == 6 * 32 * 4, "6 rows of 32 groups x 4 halfs");
+    launch_bs_layout_t<0, 6>(s, n_verts, n_shapes, layer_stride, d_records, d_dst, bs_blocks);
 }
 
-// One CTA per tile, inputs loaded straight into registers (LDG.128, L1-bypassing).
-template <int S, int LOG2C, int MINB, bool BS>
+void launch_bs_tan_layout(cudaStream_t s, uint32_t n_verts, uint32_t n_shapes, uint32_t layer_stride, const uint16_t *d_records, uint2 *d_dst,
+                          uint32_t bs_blocks)
+{
+    static_assert(kBstBlockU2 * 4 == 3 * 32 * 4, "3 rows of 32 groups x 4 halfs");
+    launch_bs_layout_t<6, 3>(s, n_verts, n_shapes, layer_stride, d_records, d_dst, bs_blocks);
+}
+
+// One CTA per tile, inputs loaded straight into registers (LDG.128, L1-bypassing).  TAN: some surface of the context has
+// tangents; whether this tile does is CTA-uniform, and a tile without them runs the same code as the TAN = false kernel.
+template <int S, int LOG2C, int MINB, bool BS, bool TAN>
 __global__ void __launch_bounds__(kBlock, MINB) k_skin(const SkinArrays sk, const SkinTile *__restrict__ tiles, const uint32_t n_tiles,
                                                      const float one, const float negzero)
 {
@@ -1212,8 +1267,18 @@ __global__ void __launch_bounds__(kBlock, MINB) k_skin(const SkinArrays sk, cons
         const float4 w0 = ld_stream(row + 6 * 32), w1 = ld_stream(row + 7 * 32), w2 = ld_stream(row + 8 * 32), w3 = ld_stream(row + 9 * 32);
         const uint4 iq = ld_stream(reinterpret_cast<const uint4 *>(row + 10 * 32));
         if (BS && T.n_shapes) apply_blend_shapes(sk, T, q, x4, y4, z4, nx4, ny4, nz4);
-        skin_quad<S, LOG2C>(s_pal, lane, x4, y4, z4, nx4, ny4, nz4, w0, w1, w2, w3, iq, reinterpret_cast<float4 *>(sk.opos) + 3 * quad,
-                            reinterpret_cast<float4 *>(sk.onrm) + 3 * quad, kc);
+        if (TAN && T.tan_blk != FYX_NONE) {
+            const uint32_t e = T.local_quad0 + q; // group within the surface
+            const float4 *trow = sk.tblk + ((size_t)T.tan_blk + (e >> 5)) * kTblkStride + (e & 31u);
+            float4 tx4 = ld_stream(trow + 0 * 32), ty4 = ld_stream(trow + 1 * 32), tz4 = ld_stream(trow + 2 * 32);
+            if (BS && T.n_shapes) apply_blend_shapes_tan(sk, T, e, tx4, ty4, tz4);
+            skin_quad<S, LOG2C, true>(s_pal, lane, x4, y4, z4, nx4, ny4, nz4, w0, w1, w2, w3, iq, reinterpret_cast<float4 *>(sk.opos) + 3 * quad,
+                                      reinterpret_cast<float4 *>(sk.onrm) + 3 * quad, kc, tx4, ty4, tz4,
+                                      reinterpret_cast<float4 *>(sk.otan) + 3 * ((size_t)T.tan_quad0 + e));
+        } else {
+            skin_quad<S, LOG2C>(s_pal, lane, x4, y4, z4, nx4, ny4, nz4, w0, w1, w2, w3, iq, reinterpret_cast<float4 *>(sk.opos) + 3 * quad,
+                                reinterpret_cast<float4 *>(sk.onrm) + 3 * quad, kc);
+        }
     }
 }
 
@@ -1551,6 +1616,25 @@ __global__ void __launch_bounds__(kBlock) k_deinterleave(const uint32_t n_verts,
     reinterpret_cast<uint32_t *>(blk)[10 * rs + j] = bi;
 }
 
+// The tangent (f32 x4 at tangent_offset; .xyz used, .w the handedness stays with the renderer) of a tangent surface →
+// its tangent blocks (fyx_internal.h).  Done once per fyx_set_skinned_tangents.  Vertex u of the surface = group u/4,
+// element u%4 of block u/128; the padding vertices up to the next multiple of 4 are zero.
+__global__ void __launch_bounds__(kBlock) k_tan_deinterleave(const uint32_t n_verts, const uint32_t n_padded, const unsigned char *d_bytes,
+                                                             const uint32_t stride, const uint32_t tangent_offset, float4 *tblk)
+{
+    const uint32_t u = blockIdx.x * kBlock + threadIdx.x;
+    if (u >= n_padded) return;
+    float t[3] = {0.f, 0.f, 0.f};
+    if (u < n_verts) {
+        const float *ft = reinterpret_cast<const float *>(d_bytes + (size_t)u * stride + tangent_offset);
+        t[0] = ft[0]; t[1] = ft[1]; t[2] = ft[2];
+    }
+    const uint32_t Q = u >> 2, j = u & 3u;
+    float *blk = reinterpret_cast<float *>(tblk + (size_t)(Q >> 5) * kTblkStride + (Q & 31)); // row 0, this group's float4
+    const size_t rs = 32 * 4; // floats between rows
+    blk[0 * rs + j] = t[0]; blk[1 * rs + j] = t[1]; blk[2 * rs + j] = t[2];
+}
+
 __global__ void __launch_bounds__(kBlock) k_ib_rows(const uint32_t n, const float *d_m16, float4 *r0, float4 *r1, float4 *r2,
                                                     uint32_t *d_err)
 {
@@ -1787,20 +1871,29 @@ void launch_palette(cudaStream_t s, const NodeArrays &a, const SkinArrays &sk)
     launch_pdl(k_palette, grid_for(sk.n_entries), kBlock, 0, s, a, sk);
 }
 
-template <int S, int LOG2C, int MINB, bool BS> static void launch_skin_t2(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles)
+template <int S, int LOG2C, int MINB, bool BS, bool TAN> static void launch_skin_t2(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles)
 {
     constexpr size_t smem_pal = (size_t)3 * S * (1 << LOG2C) * sizeof(float4);
     static bool init = false;
     if (!init) {
-        cudaFuncSetAttribute(k_skin<S, LOG2C, MINB, BS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pal);
+        cudaFuncSetAttribute(k_skin<S, LOG2C, MINB, BS, TAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pal);
         init = true;
     }
-    launch_pdl(k_skin<S, LOG2C, MINB, BS>, n_tiles, kBlock, smem_pal, s, sk, tiles, n_tiles, 1.0f, -0.0f);
+    launch_pdl(k_skin<S, LOG2C, MINB, BS, TAN>, n_tiles, kBlock, smem_pal, s, sk, tiles, n_tiles, 1.0f, -0.0f);
 }
-template <int S, int LOG2C, int MINB> static void launch_skin_t(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles, bool bs)
+// CTAs per SM the tangent instantiations are compiled for: 12 more inputs and 12 more accumulators per thread.  At 3 CTAs/SM
+// (80 registers) ptxas spills 104-128 B per thread; at 2 (116-124 registers) nothing.
+constexpr int kSkinTanMinB = 2;
+template <int S, int LOG2C, int MINB, int MINB_TAN>
+static void launch_skin_t(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles, bool bs, bool tan)
 {
-    if (bs) launch_skin_t2<S, LOG2C, MINB, true>(s, sk, tiles, n_tiles);
-    else launch_skin_t2<S, LOG2C, MINB, false>(s, sk, tiles, n_tiles);
+    if (tan) {
+        if (bs) launch_skin_t2<S, LOG2C, MINB_TAN, true, true>(s, sk, tiles, n_tiles);
+        else launch_skin_t2<S, LOG2C, MINB_TAN, false, true>(s, sk, tiles, n_tiles);
+    } else {
+        if (bs) launch_skin_t2<S, LOG2C, MINB, true, false>(s, sk, tiles, n_tiles);
+        else launch_skin_t2<S, LOG2C, MINB, false, false>(s, sk, tiles, n_tiles);
+    }
 }
 
 template <int S, int LOG2C, int STAGES, int MINB> static void launch_skin_tma_t(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles)
@@ -1842,11 +1935,11 @@ static int skin_variant()
     return v;
 }
 
-void launch_skin(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles, uint32_t max_bones, bool blend_shapes)
+void launch_skin(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, uint32_t n_tiles, uint32_t max_bones, bool blend_shapes, bool tangents)
 {
     if (!n_tiles) return;
     const int var = skin_variant();
-    if (var && max_bones <= 64 && !blend_shapes) { // the experiments cover the benchmarked palette size
+    if (var && max_bones <= 64 && !blend_shapes && !tangents) { // the experiments cover the benchmarked palette size
         if (var == 2) launch_skin_tma_t<65, 2, 2, 2>(s, sk, tiles, n_tiles);
         else if (var == 3) launch_skin_tma_t<65, 3, 3, 1>(s, sk, tiles, n_tiles);
         else if (var == 14) launch_skin2_t<65, 3, 4>(s, sk, tiles, n_tiles);
@@ -1856,11 +1949,11 @@ void launch_skin(cudaStream_t s, const SkinArrays &sk, const SkinTile *tiles, ui
     }
     // 3 CTAs/SM (<= 85 registers): capping at 64 registers for 4 CTAs/SM spills and measured 28 % slower
     if (max_bones <= 64) {       // 8 copies: 25 KB of palette planes
-        launch_skin_t<65, 3, 3>(s, sk, tiles, n_tiles, blend_shapes);
+        launch_skin_t<65, 3, 3, kSkinTanMinB>(s, sk, tiles, n_tiles, blend_shapes, tangents);
     } else if (max_bones <= 128) { // 8 copies: 50 KB
-        launch_skin_t<129, 3, 3>(s, sk, tiles, n_tiles, blend_shapes);
+        launch_skin_t<129, 3, 3, kSkinTanMinB>(s, sk, tiles, n_tiles, blend_shapes, tangents);
     } else {                       // 4 copies (2-way worst case): 49 KB
-        launch_skin_t<257, 2, 3>(s, sk, tiles, n_tiles, blend_shapes);
+        launch_skin_t<257, 2, 3, kSkinTanMinB>(s, sk, tiles, n_tiles, blend_shapes, tangents);
     }
 }
 
@@ -1958,6 +2051,13 @@ void launch_deinterleave(cudaStream_t s, uint32_t n_verts, const unsigned char *
     const uint32_t n_padded = (n_verts + 3u) & ~3u;
     if (!n_padded) return;
     k_deinterleave<<<grid_for(n_padded), kBlock, 0, s>>>(n_verts, n_padded, d_bytes, layout, n_bones, vblk, first_vertex, d_err);
+}
+
+void launch_tan_deinterleave(cudaStream_t s, uint32_t n_verts, const unsigned char *d_bytes, uint32_t stride, uint32_t tangent_offset, float4 *tblk)
+{
+    const uint32_t n_padded = (n_verts + 3u) & ~3u;
+    if (!n_padded) return;
+    k_tan_deinterleave<<<grid_for(n_padded), kBlock, 0, s>>>(n_verts, n_padded, d_bytes, stride, tangent_offset, tblk);
 }
 
 void launch_ib_rows(cudaStream_t s, uint32_t n, const float *d_m16, float4 *r0, float4 *r1, float4 *r2, uint32_t *d_err)

@@ -198,6 +198,7 @@ class Surface:
     vertex_buffer: Optional[np.ndarray] = None  # uint8, AnimatedVertex records
     surface_id: Optional[int] = None            # fyx surface id once uploaded
     blend_shapes_container: Optional[BlendShapesContainer] = None
+    skin_tangents: bool = False                 # also skin the tangents (fyx_set_skinned_tangents) for a normal-mapped renderer
     _shapes_uploaded: bool = False
 
 
@@ -529,6 +530,8 @@ class Graph:
                 bones = np.array([b.index if self.is_valid_handle(b) else L.FYX_NONE for b in s.bones], np.uint32)
                 ib = np.stack([self._records[b.index].inv_bind_pose_transform if self.is_valid_handle(b) else np.eye(4, dtype=f32).reshape(16) for b in s.bones])
                 s.surface_id = self.ctx.add_skinned_surface(i, bones, ib, s.vertex_buffer, ANIMATED_VERTEX_LAYOUT)
+                if s.skin_tangents and s.vertex_buffer is not None:  # before the blend shapes, which then lay out their tangent offsets
+                    self.ctx.set_skinned_tangents(s.surface_id, s.vertex_buffer, 32, ANIMATED_VERTEX_LAYOUT.stride)
                 self._surfaces_uploaded += 1
         self._upload_blend_shapes()
 

@@ -264,20 +264,38 @@ int32_t fyx_set_observers(fyx_ctx *ctx, uint32_t count, const fyx_observer *obse
  * standard.shader:167-173), weight = BlendShape::weight / 100 (scene/mesh/mod.rs:794-798).  `records` is the content of
  * BlendShapesContainer::blend_shape_storage as from_lists builds it (scene/mesh/surface.rs:92-218): n_shapes layers of
  * layer_stride (= width * height >= n_verts) records of 9 binary16 values — position, normal, tangent offsets of vertex
- * v at record v of the layer (tangents are not part of the skinned streams and are ignored).  `weights` = the
+ * v at record v of the layer.  The tangent offsets are laid out only for a surface that has skinned tangents at the time of
+ * the call (fyx_set_skinned_tangents, which must come first); other surfaces ignore them.  `weights` = the
  * BlendShape::weight values (0..100), NULL = 100 each (BlendShape::default()).  n_shapes = 0 removes them.
- * Costs 12 more bytes read per vertex and shape in fyx_skin; surfaces without shapes are unaffected. */
+ * Costs 12 more bytes read per vertex and shape in fyx_skin (18 on a tangent surface); surfaces without shapes are unaffected. */
 #define FYX_MAX_BLEND_SHAPES 128u /* ShaderDefinition::MAX_BLEND_SHAPE_WEIGHT_GROUPS * 4, fyrox-material/src/shader/mod.rs:616 */
 int32_t fyx_set_blend_shapes(fyx_ctx *ctx, uint32_t surface_id, uint32_t n_shapes, const void *records, uint32_t layer_stride,
                              const float *weights);
 int32_t fyx_set_blend_shape_weights(fyx_ctx *ctx, uint32_t surface_id, uint32_t n, const float *weights);
+
+/* ---- skinned tangents (opt-in, per surface) ------------------------------------------------------------------ */
+/* The standard shader skins the tangent as it skins the normal (standard.shader:197-200): acc += (mat3(P[idx_k]) * t) * w_k,
+ * after the blend shapes added offsets.tangent * weight (:167-173).  A normal-mapped renderer needs the skinned tangent for
+ * its binormal, w * cross(normal, tangent).  fyx_set_skinned_tangents adds a third skinned stream to one surface: `verts`
+ * = the surface's VertexBuffer bytes again (n_verts records of `stride` bytes) with the tangent as f32 x4 at tangent_offset
+ * (32 in AnimatedVertex); only .xyz is skinned, .w (the handedness) stays in the renderer's own vertex buffer.  Normalising,
+ * the world matrix and the binormal stay with the renderer, as for normals.  verts = NULL turns the surface's tangents off.
+ * FYX_ERR_INVALID_ARGUMENT: stride or tangent_offset not a multiple of 4, or tangent_offset + 16 > stride.
+ * FYX_ERR_STATE: the surface already has blend shapes (call this before fyx_set_blend_shapes).  Surfaces without tangents
+ * run exactly as before; the tangent data belongs to the surface and survives fyx_set_topology.  Costs 12 bytes read and
+ * 12 written per vertex of a tangent surface in fyx_skin. */
+int32_t fyx_set_skinned_tangents(fyx_ctx *ctx, uint32_t surface_id, const void *verts, uint32_t stride, uint32_t tangent_offset);
+/* The skinned tangents of the last fyx_skin / render prep, packed xyz (n_verts*3); FYX_ERR_STATE for a surface without tangents. */
+int32_t fyx_get_skinned_tangents(fyx_ctx *ctx, uint32_t surface_id, float *out_tan3);
+int32_t fyx_get_skinned_tangents_device(fyx_ctx *ctx, uint32_t surface_id, const float **d_tan3);
 
 /* SurfaceInstanceData::bone_matrices for every skinned surface (scene/mesh/mod.rs:781-793):
  * P[k] = bone_k.global_transform * bone_k.inv_bind_pose_transform; dead / FYX_NONE bone ⇒ identity. */
 int32_t fyx_build_palettes(fyx_ctx *ctx);
 /* Linear-blend skinning of every skinned surface: positions as Mesh::accurate_world_bounding_box
  * (scene/mesh/mod.rs:501-522), normals as the standard shader (fyrox-material/src/shader/standard/opengl/
- * standard.shader:192-195) — into device-resident position / normal streams. */
+ * standard.shader:192-195) — into device-resident position / normal streams; and the tangents of the surfaces that have
+ * them (fyx_set_skinned_tangents, standard.shader:197-200) into a third stream. */
 int32_t fyx_skin(fyx_ctx *ctx);
 
 /* One whole frame of render prep, in stream order, with one host synchronisation at the end:
